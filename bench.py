@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the WaveNet inference hot path (contract: see DESIGN.md §7).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2], "C3"): fp16, 20 layers, R64/S256/A256, maxDilation 512,
@@ -324,6 +324,19 @@ def reference_gpu_kernels(args, our_khz, n_samples=600):
         return {"unavailable": str(ex)[:200]}
 
 
+def dump_outputs(out_dir, name, y, max_bytes):
+    """Writes the sampled indices y [utterances][samples] as out_dir/<name>.npy in float32 (exact below 2**24).  When that
+    exceeds max_bytes, only a fixed, seeded sample of whole utterances is written, and their indices as <name>_rows.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    keep = max(1, max_bytes // (4 * y.shape[1]))
+    if keep < y.shape[0]:
+        rows = np.sort(np.random.Generator(np.random.PCG64(SEED)).choice(y.shape[0], keep, replace=False))
+        y = y[rows]
+        np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, name + ".npy"), y.astype(np.float32))
+
+
 # --------------------------------------------------------------------------- our arm
 def run_ours(args, rank, world, local_rank):
     import numpy as np
@@ -421,6 +434,10 @@ def run_ours(args, rank, world, local_rank):
     ev1.record(stream)
     barrier()
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs:                   # before the e2e leg below overwrites the conditioning the timed steps ran on
+        y = np.zeros((B, N), np.int32)
+        eng.get_yout(y, 0, N, stream); torch.cuda.synchronize()
+        dump_outputs(args.dump_outputs, "yout" if world == 1 else f"yout_rank{rank}", y, (64 << 20) // world)
     elapsed_ms = ev0.elapsed_time(ev1)
     kernel_ms = statistics.mean(a.elapsed_time(b) for a, b in kev)
     info = eng.launch_info()
@@ -546,7 +563,11 @@ def main():
     ap.add_argument("--e2e-chunk", type=int, default=1000)
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's sampled indices (yOut) as DIR/yout.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     MODEL.clear(); MODEL.update(CONFIGS[args.config])
     if args.batch is None:
         args.batch = MODEL["batch"]

@@ -16,6 +16,10 @@ it replays the test's inputs with the reference's own Matrix::randomize + libc r
     <key>/xt_last    float32 [2][B][R] last layer output, /skip_last float32 [2][B][S]
 
 Inputs are not stored (tests/refgen.py regenerates them bit-exactly; in_sha proves it).
+
+It also writes reference_cpu_fresh.npz: for the fresh shapes of tests/test_oracle_pin.py (synthetic and lively
+inputs, FRESH_ITERS runs each), <key>/in_sha and, per run, <key>/y int32 [batch][N] and the last-sample
+activations <key>/xt [L][B][R], /skip [L][B][S], /zs, /za, /p [B][A].
 """
 import hashlib
 import os
@@ -68,5 +72,29 @@ def main():
     print("wrote", path, os.path.getsize(path), "bytes")
 
 
+def fresh():
+    from tests import test_oracle_pin as pin
+    out = {}
+    for shape in pin.FRESH_SHAPES:
+        R, S, A, L, B, bs, N, md = shape
+        for gen in pin.FRESH_GENS:
+            w = pin.fresh_inputs(shape, gen)
+            ref = po.RefCPU(L, B, N, R, S, A, md)
+            ref.load(w)
+            ref.set_inputs(w["Lh"], w["selectors"])
+            key = pin.fresh_key(shape, gen)
+            runs = []
+            for _ in range(pin.FRESH_ITERS):
+                y = ref.run(N, bs)
+                runs.append(dict(ref.activations(), y=y))
+            out[key + "/in_sha"] = np.array(sha([w[k] for k in INPUT_KEYS]))
+            for k in runs[0]:
+                out[f"{key}/{k}"] = np.stack([r[k] for r in runs])
+            print(key, "ok")
+    np.savez_compressed(pin.FRESH_GOLDEN, **out)
+    print("wrote", pin.FRESH_GOLDEN, os.path.getsize(pin.FRESH_GOLDEN), "bytes")
+
+
 if __name__ == "__main__":
     main()
+    fresh()

@@ -1,10 +1,12 @@
 """bench.py's JSON contract, exercised on the CPU through the reference arm (`--impl reference` times the reference's
-own CPU model, oracle/_ref, on a bounded sample): one JSON line with the keys the driver reads."""
+own CPU model, oracle/_ref, on a bounded sample): one JSON line with the keys the driver reads.  And --dump-outputs: what
+the timed path computed, written so that two runs or two builds can be compared."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -29,6 +31,38 @@ def test_reference_arm_prints_one_contract_line():
     assert cb["kind"] == "reference" and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
     e2e = d["e2e"]
     assert e2e["value"] == d["value"] and e2e["unit"] == d["unit"] and e2e["h2d_bytes_per_step"] == 0 and e2e["d2h_bytes_per_step"] == 0
+
+
+def test_dump_outputs_keeps_a_fixed_sample_of_utterances_past_the_size_limit(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    y = np.arange(10 * 6, dtype=np.int32).reshape(10, 6)
+    bench.dump_outputs(str(tmp_path / "all"), "yout", y, 10 * 6 * 4)
+    whole = np.load(tmp_path / "all" / "yout.npy")
+    assert whole.dtype == np.float32 and np.array_equal(whole, y) and not (tmp_path / "all" / "yout_rows.npy").exists()
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), "yout", y, 4 * 6 * 4 + 5)
+    rows = np.load(tmp_path / "a" / "yout_rows.npy")
+    assert rows.dtype == np.float64 and len(rows) == 4 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "yout.npy"), y[rows.astype(int)])
+    assert np.array_equal(rows, np.load(tmp_path / "b" / "yout_rows.npy"))
+
+
+@pytest.mark.gpu
+def test_our_arm_dumps_the_same_outputs_from_run_to_run(tmp_path):
+    """--dump-outputs writes the last timed step's yOut; with the same arguments two runs sample the same indices."""
+    lines = []
+    for d in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "1", "--samples", "1000",
+                              "--no-extra", "--no-cpu", "--no-e2e", "--dump-outputs", str(tmp_path / d)],
+                             capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines.append(json.loads(out.stdout.strip().splitlines()[-1]))
+    assert lines[0]["steps"] == 3 and lines[0]["value"] > 0
+    ya, yb = np.load(tmp_path / "a" / "yout.npy"), np.load(tmp_path / "b" / "yout.npy")
+    assert ya.dtype == np.float32 and ya.shape == (lines[0]["config"]["batch_per_gpu"], 1000)
+    assert ya.min() >= 0 and ya.max() < 256 and len(np.unique(ya)) > 16
+    assert np.array_equal(ya, yb)
 
 
 def test_reference_arm_nonzero_ranks_exit_quietly():

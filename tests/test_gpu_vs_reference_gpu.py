@@ -1,16 +1,39 @@
-"""Parity against the reference's OWN CUDA kernels (oracle/_ref/ref_gpu_harness: unmodified nv_wavenet.cuh + the
-PERSISTENT kernel, rebuilt for sm_100a) -- BASELINE.json north_star: "bit-exact sampled indices in fp32, softmax
-logits within 1e-2 rel in fp16".  Skipped where the harness was not built."""
+"""Parity against the reference's OWN CUDA kernels (unmodified nv_wavenet.cuh + the PERSISTENT kernel, rebuilt for sm_100a
+as oracle/_ref/ref_gpu_harness) -- BASELINE.json north_star: "bit-exact sampled indices in fp32, softmax logits within 1e-2
+rel in fp16".  What those kernels computed on the inputs below is stored in tests/golden/reference_gpu.npz
+(tests/golden/make_golden_ref_gpu.py)."""
+import os
+
 import numpy as np
 import pytest
 
 import nv_wavenet_b200 as nw
-from oracle import ref_gpu
-from tests import refgen
+from tests import common, refgen
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_gpu.available(), reason="oracle/_ref/ref_gpu_harness not built")]
+pytestmark = pytest.mark.gpu
 
 R, S, A, L, MD = 64, 256, 256, 20, 8
+GOLDEN = os.path.join(common.HERE, "golden", "reference_gpu.npz")
+
+
+def fp32_case():
+    """(inputs, B, N) at the reference test's scale (nv_wavenet_test.cu:36-48)."""
+    B, N = 16, 8
+    return refgen.reference_test_inputs(refgen.GlibcRand(30), R, S, A, L, B, N), B, N
+
+
+def fp16_case():
+    B, N = 16, 6
+    w = refgen.lively_inputs(4, R, S, A, L, B, N)
+    for k in ("Wprev", "Wcur", "Wres", "Wskip", "Wzs", "Wza", "embPrev", "embCur", "Lh"):
+        w[k] = (w[k] * 0.6).astype(np.float32)          # keep the reference's fp16 ACCUMULATION (matrix_math.cuh:119-157) well conditioned
+    return w, B, N
+
+
+def _golden(name, w):
+    g = np.load(GOLDEN)
+    assert common.sha([w[k] for k in common.INPUT_KEYS]) == str(g[name + "/in_sha"]), "inputs differ from the stored run's"
+    return {k: g[f"{name}/{k}"] for k in ("y", "za")}
 
 
 def _ours(w, B, N, dtype, forced=None):
@@ -27,10 +50,8 @@ def test_fp32_indices_equal_reference_gpu_kernel():
     """Same weights / Lh / selectors through the reference PERSISTENT kernel and through ours: every sampled index equal
     (reference test scale, nv_wavenet_test.cu:36-48; the reference kernel uses fast-math, so agreement is what its own
     test asserts against the CPU model -- we hold the CPU model bit-exactly)."""
-    B, N = 16, 8
-    rng = refgen.GlibcRand(30)
-    w = refgen.reference_test_inputs(rng, R, S, A, L, B, N)
-    ref = ref_gpu.run(w, 32, R, S, A, L, MD, B, N, mode=3, chunk=7)
+    w, B, N = fp32_case()
+    ref = _golden("fp32", w)
     y, za, p = _ours(w, B, N, nw.FP32)
     assert np.array_equal(y, ref["y"])
     assert np.all(np.abs(za - ref["za"]) <= 1e-4 * np.abs(ref["za"]) + 1e-6)
@@ -39,11 +60,8 @@ def test_fp32_indices_equal_reference_gpu_kernel():
 def test_fp16_logits_within_1e2_of_reference_fp16_kernel():
     """fp16: trajectories of two different fp16 pipelines diverge, so both are compared at matched history: ours is
     teacher-forced with the reference kernel's own samples; logits of the last sample within 1e-2."""
-    B, N = 16, 6
-    w = refgen.lively_inputs(4, R, S, A, L, B, N)
-    for k in ("Wprev", "Wcur", "Wres", "Wskip", "Wzs", "Wza", "embPrev", "embCur", "Lh"):
-        w[k] = (w[k] * 0.6).astype(np.float32)          # keep the reference's fp16 ACCUMULATION (matrix_math.cuh:119-157) well conditioned
-    ref = ref_gpu.run(w, 16, R, S, A, L, MD, B, N, mode=3, chunk=2048)
+    w, B, N = fp16_case()
+    ref = _golden("fp16", w)
     y, za, p = _ours(w, B, N, nw.FP16, forced=ref["y"])
     scale = np.abs(ref["za"]).max(axis=1, keepdims=True)
     err = np.abs(za - ref["za"])

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 from tests import refgen
-from tests.test_cond_producer import GOLD, host_cond
+from tests.test_cond_producer import GOLD, golden_lh, host_cond
 
 pytestmark = pytest.mark.gpu
 
@@ -70,12 +70,12 @@ def test_device_conditioning_store_matches_reference_module(kernel, monkeypatch)
     assert n == T * stride
     lib = _lib.lib()
     lib.nvwn_debug_get_conditioning.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
-    got = np.full((n, L, B, 2 * R), np.nan, np.float32)
-    assert lib.nvwn_debug_get_conditioning(e._h, C.c_void_p(got.ctypes.data), first, n) == 0
-    want = GOLD["c_Lh"]
+    full = np.full((n, L, B, 2 * R), np.nan, np.float32)
+    assert lib.nvwn_debug_get_conditioning(e._h, C.c_void_p(full.ctypes.data), first, n) == 0
+    got, want = golden_lh(full, "c")
     scale = np.abs(want).max()
     tol = 1e-5 if kernel == "fp32" else 1e-3
-    assert np.isfinite(got).all() and np.abs(got - want).max() <= tol * scale, np.abs(got - want).max() / scale
+    assert np.isfinite(full).all() and np.abs(got - want).max() <= tol * scale, np.abs(got - want).max() / scale
 
 
 def test_out_of_range_is_rejected():

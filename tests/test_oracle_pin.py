@@ -7,8 +7,11 @@
    oracle/_ref = the reference's nv_wavenet_reference.cpp compiled unmodified).
 3. The oracle in PORTABLE-math mode (the arithmetic contract the CUDA fp32 kernel implements
    bit-exactly) samples identical indices and stays within a few ulp on activations.
-4. Where oracle/_ref is present, the same on fresh shapes/seeds directly against the reference.
+4. The same on fresh shapes/seeds, against the reference CPU model's outputs on them (golden vectors
+   made by tests/golden/make_golden.py, as in 2).
 """
+import os
+
 import numpy as np
 import pytest
 
@@ -80,28 +83,43 @@ def test_portable_math_accuracy():
     assert lib.wno_round_fp16(1.0009765625 + 1e-4) == np.float32(np.float16(1.0009765625 + 1e-4))
 
 
-needs_ref = pytest.mark.skipif(not po.have_ref(), reason="oracle/_ref not built (no /root/reference here)")
-
-
-@needs_ref
-@pytest.mark.parametrize("shape", [
+FRESH_SHAPES = [
     # R, S, A, L, B(max), batch, N, maxDil
     (32, 128, 256, 6, 3, 3, 20, 4),
     (64, 256, 256, 5, 4, 4, 12, 8),       # (the reference CPU model asserts batch_size == max_batch, reference.cpp:72)
     (64, 128, 512, 3, 1, 1, 40, 16),
     (128, 256, 256, 2, 2, 2, 6, 2),
-])
-@pytest.mark.parametrize("gen", ["uniform", "lively"])
-def test_oracle_vs_reference_cpu_fresh_shapes(shape, gen):
+]
+FRESH_GENS = ["uniform", "lively"]
+FRESH_ITERS = 2
+FRESH_GOLDEN = os.path.join(common.HERE, "golden", "reference_cpu_fresh.npz")
+
+
+def fresh_inputs(shape, gen):
     R, S, A, L, B, bs, N, md = shape
-    w = (refgen.synthetic_inputs if gen == "uniform" else refgen.lively_inputs)(1234 + R + N, R, S, A, L, B, N)
-    ref = po.RefCPU(L, B, N, R, S, A, md); ref.load(w); ref.set_inputs(w["Lh"], w["selectors"])
+    return (refgen.synthetic_inputs if gen == "uniform" else refgen.lively_inputs)(1234 + R + N, R, S, A, L, B, N)
+
+
+def fresh_key(shape, gen):
+    return "_".join(str(v) for v in shape) + "_" + gen
+
+
+@pytest.mark.parametrize("shape", FRESH_SHAPES)
+@pytest.mark.parametrize("gen", FRESH_GENS)
+def test_oracle_vs_reference_cpu_fresh_shapes(shape, gen):
+    """Against what the reference CPU model computed on the same inputs (stored by tests/golden/make_golden.py)."""
+    R, S, A, L, B, bs, N, md = shape
+    w = fresh_inputs(shape, gen)
+    key = fresh_key(shape, gen)
+    g = np.load(FRESH_GOLDEN)
+    assert common.sha([w[k] for k in common.INPUT_KEYS]) == str(g[key + "/in_sha"])
     o = po.Oracle(L, B, N, R, S, A, md, math=po.MATH_LIBM); o.load(w); o.set_inputs(w["Lh"], w["selectors"])
     p = po.Oracle(L, B, N, R, S, A, md, math=po.MATH_PORTABLE); p.load(w); p.set_inputs(w["Lh"], w["selectors"])
-    for _ in range(2):
-        yr, yo, yp = ref.run(N, bs), o.run(N, bs), p.run(N, bs)
+    for it in range(FRESH_ITERS):
+        yr, yo, yp = g[key + "/y"][it], o.run(N, bs), p.run(N, bs)
         assert np.array_equal(yr, yo)
-        ar, ao, ap = ref.activations(), o.activations(), p.activations()
+        ar = {k: g[f"{key}/{k}"][it] for k in ("xt", "skip", "zs", "za", "p")}
+        ao, ap = o.activations(), p.activations()
         for k in ar:
             assert common.bits_equal(ar[k][:, :bs], ao[k][:, :bs]) if ar[k].ndim == 3 else common.bits_equal(ar[k][:bs], ao[k][:bs])
         if np.array_equal(yr, yp):
