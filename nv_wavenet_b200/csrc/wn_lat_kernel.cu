@@ -453,7 +453,7 @@ __global__ void __launch_bounds__(NT, 1) wn_lat_kernel(const WnParams p, const u
                     mbar_arrive_a(s_pfull + 8 * slot3);
                 } else {
                     int sl = itp.slot - d; if (sl < 0) sl += slots;
-                    cp_async16(dst, gring - lane16 + (size_t)((uint32_t)(sl * L + itp.l) * rstride) + (size_t)(w * 32 + lane) * 16);
+                    cp_async16(dst, gring - lane16 + (size_t)(sl * L + itp.l) * rstride + (size_t)(w * 32 + lane) * 16);
                     cp_async_arrive_noinc(s_pfull + 8 * slot3);
                 }
             }
@@ -588,7 +588,7 @@ __global__ void __launch_bounds__(NT, 1) wn_lat_kernel(const WnParams p, const u
             if (l + 1 < L) {
                 const uint32_t x01 = pack_h2(xres[0], xres[1]), x23 = pack_h2(xres[2], xres[3]);
                 sts64(sm + C::O_XBUF + xchg, x01, x23);
-                stg_v2(gring + (size_t)((uint32_t)(it0.slot * L + l + 1) * rstride) + jw * 512 + hw * 8, x01, x23);
+                stg_v2(gring + (size_t)(it0.slot * L + l + 1) * rstride + jw * 512 + hw * 8, x01, x23);
             }
             if (tid == 0) TRACE(0, 14);
             if (DUMP) {
@@ -651,7 +651,7 @@ __global__ void __launch_bounds__(NT, 1) wn_lat_kernel(const WnParams p, const u
                 }
                 const uint32_t x01 = pack_h2(xres[0], xres[1]), x23 = pack_h2(xres[2], xres[3]);
                 sts64(sm + C::O_XBUF + xchg, x01, x23);
-                stg_v2(gring + (size_t)((uint32_t)(it0.slot * L) * rstride) + jw * 512 + hw * 8, x01, x23);
+                stg_v2(gring + (size_t)(it0.slot * L) * rstride + jw * 512 + hw * 8, x01, x23);
                 // previous-index rows of the NEXT sample (= this sample's current index): global -> shared, asynchronously
                 const unsigned char* ep = static_cast<const unsigned char*>(p.embPrev);
                 const uint32_t en = sm + C::O_EPBUF + (epar ^ 1) * (TU * EROW * 4);
@@ -741,7 +741,7 @@ __global__ void __launch_bounds__(NT, 1) wn_lat_kernel(const WnParams p, const u
             // ---------------- softmax + categorical sample (matrix.cpp:167-183, reference.cpp:106-121): warp w serves
             // utterances 2w and 2w+1; lane holds 8 consecutive classes of each
             {
-                float e[2][8], m[2] = {0.f, 0.f};                          // the reference starts the max at 0 (matrix.cpp:171)
+                float e[2][8], m[2] = {-INFINITY, -INFINITY};              // the true row max (DESIGN.md §3)
 #pragma unroll
                 for (int r = 0; r < 2; r++) {
                     const uint4 u0 = lds128(sm + C::O_LBUF + ((2 * w + r) * LROW + 8 * lane) * 4), u1 = lds128(sm + C::O_LBUF + ((2 * w + r) * LROW + 8 * lane + 4) * 4);
@@ -1044,7 +1044,7 @@ __global__ void __launch_bounds__(NTC, 1) wn_lat2_kernel(const WnParams p, const
                     }
                     const uint32_t x01 = pack_h2(xres[0], xres[1]), x23 = pack_h2(xres[2], xres[3]);
                     sts64(sm + M::C_XBUF + xchg, x01, x23);
-                    stg_v2(gring + lane16 + (size_t)((uint32_t)(it0.slot * L) * rstride) + jw * 512 + hw * 8, x01, x23);
+                    stg_v2(gring + lane16 + (size_t)(it0.slot * L) * rstride + jw * 512 + hw * 8, x01, x23);
                     const unsigned char* ep = static_cast<const unsigned char*>(p.embPrev);
                     const uint32_t en = sm + M::C_EPBUF + (epar ^ 1) * (TU * EROW * 4);
                     cp_async4(en + (g * EROW + 4 * w + t4) * 4, ep + (size_t)yc0 * 128 + (4 * w + t4) * 4);
@@ -1099,7 +1099,7 @@ __global__ void __launch_bounds__(NTC, 1) wn_lat2_kernel(const WnParams p, const
                     if (l + 1 < L) {
                         const uint32_t x01 = pack_h2(xres[0], xres[1]), x23 = pack_h2(xres[2], xres[3]);
                         sts64(sm + M::C_XBUF + xchg, x01, x23);
-                        stg_v2(gring + lane16 + (size_t)((uint32_t)(it0.slot * L + l + 1) * rstride) + jw * 512 + hw * 8, x01, x23);
+                        stg_v2(gring + lane16 + (size_t)(it0.slot * L + l + 1) * rstride + jw * 512 + hw * 8, x01, x23);
                     }
                     TRACE2(0, 14);
                     if (DUMP) {
@@ -1257,7 +1257,7 @@ __global__ void __launch_bounds__(NTC, 1) wn_lat2_kernel(const WnParams p, const
                 bar_compute();
                 TRACE2(1, 22);
                 {   // softmax + categorical sample: warp w serves utterances 2w and 2w+1; lane holds 8 consecutive classes of each
-                    float e[2][8], m[2] = {0.f, 0.f};
+                    float e[2][8], m[2] = {-INFINITY, -INFINITY};          // the true row max (DESIGN.md §3)
 #pragma unroll
                     for (int r = 0; r < 2; r++) {
                         const uint4 u0 = lds128(sm + M::T_LBUF + ((2 * w + r) * LROW + 8 * lane) * 4), u1 = lds128(sm + M::T_LBUF + ((2 * w + r) * LROW + 8 * lane + 4) * 4);
@@ -1375,7 +1375,7 @@ __global__ void __launch_bounds__(NTC, 1) wn_lat2_kernel(const WnParams p, const
                         mbar_arrive_a(s_pfull + 8 * slot);
                     } else {
                         int sl = itp.slot - d; if (sl < 0) sl += slots;
-                        cp_async16(dst, gring + (size_t)((uint32_t)(sl * L + itp.l) * rstride) + (size_t)(w * 32 + lane) * 16);
+                        cp_async16(dst, gring + (size_t)(sl * L + itp.l) * rstride + (size_t)(w * 32 + lane) * 16);
                         cp_async_arrive_noinc(s_pfull + 8 * slot);
                     }
                 }

@@ -32,6 +32,7 @@ namespace {
 template <typename TD> struct Num;
 template <> struct Num<float> {
     static constexpr bool exact = true;
+    static constexpr bool true_max = false;
     static __device__ __forceinline__ float ld(const float* p) { return __ldg(p); }
     static __device__ __forceinline__ float ldcg(const float* p) { return __ldcg(p); }
     static __device__ __forceinline__ void st(float* p, float v) { *p = v; }
@@ -44,6 +45,7 @@ template <> struct Num<float> {
 };
 template <> struct Num<__half> {
     static constexpr bool exact = false;
+    static constexpr bool true_max = true;      // softmax from the true row max, not from max(0, logits) as the reference does
     static __device__ __forceinline__ float ld(const __half* p) { return __half2float(__ldg(p)); }
     static __device__ __forceinline__ float ldcg(const __half* p) { return __half2float(__ldcg(p)); }
     static __device__ __forceinline__ void st(__half* p, float v) { *p = __float2half_rn(v); }
@@ -61,6 +63,7 @@ template <> struct Num<__half> {
 // class boundary; nv_wavenet_test.cu:273-298 tolerances on the activations) -- but free of the 8-cycle-per-term serial chain.
 struct NumFast32 {
     static constexpr bool exact = false;
+    static constexpr bool true_max = false;     // the reference GPU kernels' softmax, max starting at 0
     static __device__ __forceinline__ float ld(const float* p) { return __ldg(p); }
     static __device__ __forceinline__ float ldcg(const float* p) { return __ldcg(p); }
     static __device__ __forceinline__ void st(float* p, float v) { *p = v; }
@@ -551,7 +554,7 @@ __global__ void __launch_bounds__(Shape<R, S>::NT + (RING ? 32 : 0), 1) wn_strea
             if (warp < BT) {
                 const int per = A / 32;
                 const float* z = za + warp * A + lane * per;
-                float mx = 0.f;
+                float mx = N::true_max ? -INFINITY : 0.f;          // fp16: the true row max (DESIGN.md §3)
                 for (int j = 0; j < per; j++) mx = fmaxf(mx, z[j]);
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));

@@ -1065,14 +1065,14 @@ __global__ void __launch_bounds__(NT, 1) wn_tc_kernel(const WnParams p, const un
             // ---------------- Za, softmax, categorical sample   (reference.cpp:100-121)
             // The two threads of an utterance each take 128 logits: a first TMEM pass finds the local max in fp32, a second one parks
             // (z - max) as fp16 in the thread's own row of the (now dead) activation tiles -- the rounding error is proportional to the
-            // distance from the max, i.e. negligible where the probability mass is; exp / sums / scan run from shared memory; the
+            // distance from the row's true max, i.e. negligible where the probability mass is; exp / sums / scan run from shared memory; the
             // halves meet through s_pair (local max, local sum) and s_y.
             mbar_wait(out_full, ph_out); ph_out ^= 1;
             tc_fence_after_sync();
             if (tid == tr_tid) TRACE(0, 10);
             constexpr int PART = A / NS, NCH = PART / 16;               // logits per thread, 16-logit chunks per thread
             const int a_lo = sub * PART;
-            float mx = 0.f;                                             // matrix.cpp:171 starts the max at 0
+            float mx = -INFINITY;                                       // the true row max (DESIGN.md §3)
             float csum[NCH];
             float lsum = 0.f;
             auto expz = [&](uint32_t packed, float& e0, float& e1) {       // packed = (z - local max) in fp16
@@ -1130,7 +1130,7 @@ __global__ void __launch_bounds__(NT, 1) wn_tc_kernel(const WnParams p, const un
             int y = A - 1;
             if (wv) {
                 float pm[NS], ps[NS];
-                float M = 0.f;
+                float M = -INFINITY;
 #pragma unroll
                 for (int i = 0; i < NS; i++) { pm[i] = s_pair[(u * NS + i) * 2]; ps[i] = s_pair[(u * NS + i) * 2 + 1]; M = fmaxf(M, pm[i]); }
                 float total = 0.f, off = 0.f, fme = 1.f, mine_hi = 0.f;

@@ -98,11 +98,29 @@ float wno_sigmoidf_portable(float x)
     return 1.0f / den;
 }
 
-float wno_round_fp16(float x)
+/* (float)(_Float16)x, round to nearest even, in integer arithmetic: the compiler's conversion is a library call on x86-64
+ * without F16C, and the fp16-contract model rounds every weight of every dot product (equal for all 2^32 inputs). */
+static inline float round_fp16(float x)
 {
-    _Float16 h = (_Float16)x;
-    return (float)h;
+    uint32_t u, a, s;
+    float r;
+    memcpy(&u, &x, 4);
+    a = u & 0x7FFFFFFFu; s = u & 0x80000000u;
+    if (a >= 0x7F800000u) return x;                                   /* inf, nan */
+    if (a >= 0x477FF000u) u = s | 0x7F800000u;                        /* rounds past 65504 */
+    else if (a >= 0x38800000u) u = s | ((a + 0x0FFFu + ((a >> 13) & 1u)) & ~0x1FFFu);    /* normal: 11 significant bits */
+    else {                                                            /* subnormal: a multiple of 2^-24, the ulp of [0.5, 1) */
+        float m;
+        memcpy(&m, &a, 4);
+        m = (m + 0.5f) - 0.5f;
+        memcpy(&u, &m, 4);
+        u |= s;
+    }
+    memcpy(&r, &u, 4);
+    return r;
 }
+
+float wno_round_fp16(float x) { return round_fp16(x); }
 
 /* ------------------------------------------------------------------------- */
 
@@ -221,19 +239,29 @@ static inline float m_exp(const wno_model* m, float x) { return m->math_mode == 
 static inline float m_tanh(const wno_model* m, float x) { return m->math_mode == WNO_MATH_LIBM ? tanhf(x) : wno_tanhf_portable(x); }
 /* ref: nv_wavenet_reference.cpp:36 */
 static inline float m_sigmoid(const wno_model* m, float x) { return 1.f / (1.f + m_exp(m, -x)); }
-static inline float q16(const wno_model* m, float x) { return m->prec_mode == WNO_PREC_FP16 ? wno_round_fp16(x) : x; }
+static inline float q16(const wno_model* m, float x) { return m->prec_mode == WNO_PREC_FP16 ? round_fp16(x) : x; }
 
 /* ref: matrix.cpp:85-102 matrix_multiply, one output element.
- * W is M x K col-major; x has K contiguous elements.  wq/xq: round operands to fp16 first. */
-static inline float dot_row(const wno_model* m, const float* W, int M, int K, int row, const float* x)
+ * W is M x K col-major; x has K contiguous elements.  In PREC_FP16 both operands arrive rounded to fp16 (see wno_run). */
+static inline float dot_row(const float* W, int M, int K, int row, const float* x)
 {
     float sum = 0;
-    if (m->prec_mode == WNO_PREC_FP16) {
-        for (int k = 0; k < K; k++) sum += wno_round_fp16(W[row + (size_t)k * M]) * wno_round_fp16(x[k]);
-    } else {
-        for (int k = 0; k < K; k++) sum += W[row + (size_t)k * M] * x[k];
-    }
+    for (int k = 0; k < K; k++) sum += W[row + (size_t)k * M] * x[k];
     return sum;
+}
+
+/* PREC_FP16 operands: the weights rounded once per run, an activation vector once per use (into buf) */
+static float* rounded_copy(const float* W, size_t n)
+{
+    float* q = fzalloc(n);
+    for (size_t i = 0; i < n; i++) q[i] = round_fp16(W[i]);
+    return q;
+}
+static inline const float* q16v(const wno_model* m, const float* x, int n, float* buf)
+{
+    if (m->prec_mode != WNO_PREC_FP16) return x;
+    for (int i = 0; i < n; i++) buf[i] = round_fp16(x[i]);
+    return buf;
 }
 
 int wno_run(wno_model* m, int num_samples, int batch_size, int* yOut)
@@ -243,6 +271,14 @@ int wno_run(wno_model* m, int num_samples, int batch_size, int* yOut)
     int status = 0;
     float* a_prev = fzalloc(2 * R); float* a_cur = fzalloc(2 * R); float* hp = fzalloc(2 * R);
     float* h = fzalloc(R); float* zeroR = fzalloc(R); float* skipv = fzalloc(S); float* zs = fzalloc(A);
+    float* qa = fzalloc(R); float* qb = fzalloc(R); float* qh = fzalloc(R); float* qs = fzalloc(S); float* qz = fzalloc(A);
+    const float *Wprev = m->Wprev, *Wcur = m->Wcur, *Wres = m->Wres, *Wskip = m->Wskip, *Wzs = m->Wzs, *Wza = m->Wza;
+    float* wq[6] = {NULL, NULL, NULL, NULL, NULL, NULL};
+    if (m->prec_mode == WNO_PREC_FP16) {
+        Wprev = wq[0] = rounded_copy(m->Wprev, (size_t)L * 2 * R * R); Wcur = wq[1] = rounded_copy(m->Wcur, (size_t)L * 2 * R * R);
+        Wres = wq[2] = rounded_copy(m->Wres, (size_t)L * R * R); Wskip = wq[3] = rounded_copy(m->Wskip, (size_t)L * S * R);
+        Wzs = wq[4] = rounded_copy(m->Wzs, (size_t)A * S); Wza = wq[5] = rounded_copy(m->Wza, (size_t)A * A);
+    }
 
     for (int t = 0; t < num_samples; t++) {
         float* ring_t = m->ring + (size_t)(t % slots) * (L + 1) * B * R;
@@ -262,12 +298,14 @@ int wno_run(wno_model* m, int num_samples, int batch_size, int* yOut)
                 dilation *= 2;
                 if (dilation > m->maxDil) dilation = 1;
                 /* ref: nv_wavenet_reference.cpp:59-72 nvWavenetLayer, pre-activation */
-                const float* Wp = m->Wprev + (size_t)l * 2 * R * R;
-                const float* Wc = m->Wcur + (size_t)l * 2 * R * R;
+                const float* Wp = Wprev + (size_t)l * 2 * R * R;
+                const float* Wc = Wcur + (size_t)l * 2 * R * R;
                 const float* lh = m->Lh + (((size_t)t * L + l) * B + b) * 2 * R;
+                const float* xtmd_q = q16v(m, xtmd, R, qa);
+                const float* xin_q = q16v(m, xin, R, qb);
                 for (int row = 0; row < 2 * R; row++) {
-                    a_prev[row] = dot_row(m, Wp, 2 * R, R, row, xtmd);
-                    a_cur[row] = dot_row(m, Wc, 2 * R, R, row, xin);
+                    a_prev[row] = dot_row(Wp, 2 * R, R, row, xtmd_q);
+                    a_cur[row] = dot_row(Wc, 2 * R, R, row, xin_q);
                     float v = a_prev[row] + a_cur[row];
                     v = v + q16(m, m->Bh[(size_t)l * 2 * R + row]);
                     v = v + q16(m, lh[row]);
@@ -275,22 +313,23 @@ int wno_run(wno_model* m, int num_samples, int batch_size, int* yOut)
                 }
                 /* ref: nv_wavenet_reference.cpp:74-80 gate */
                 for (int r = 0; r < R; r++) h[r] = m_tanh(m, hp[r]) * m_sigmoid(m, hp[r + R]);
+                const float* h_q = q16v(m, h, R, qh);
                 /* ref: nv_wavenet_reference.cpp:82-84 residual */
-                const float* Wr = m->Wres + (size_t)l * R * R;
+                const float* Wr = Wres + (size_t)l * R * R;
                 float* xout = ring_t + ((size_t)(l + 1) * B + b) * R;
                 for (int r = 0; r < R; r++) {
-                    float v = dot_row(m, Wr, R, R, r, h);
+                    float v = dot_row(Wr, R, R, r, h_q);
                     v = v + q16(m, m->Bres[(size_t)l * R + r]);
                     v = v + xin[r];
                     xout[r] = v;
                     m->xtOut[((size_t)l * B + b) * R + r] = v;
                 }
                 /* ref: nv_wavenet_reference.cpp:86-90 skip accumulate (+relu on the last layer) */
-                const float* Ws = m->Wskip + (size_t)l * S * R;
+                const float* Ws = Wskip + (size_t)l * S * R;
                 float* so = m->skipOut + ((size_t)l * B + b) * S;
                 const float* si = l ? m->skipOut + ((size_t)(l - 1) * B + b) * S : NULL;
                 for (int s = 0; s < S; s++) {
-                    float v = dot_row(m, Ws, S, R, s, h);
+                    float v = dot_row(Ws, S, R, s, h_q);
                     v = v + (si ? si[s] : 0.f);
                     v = v + q16(m, m->Bskip[(size_t)l * S + s]);
                     if (l == L - 1) v = (v < 0) ? 0.f : v;
@@ -301,14 +340,16 @@ int wno_run(wno_model* m, int num_samples, int batch_size, int* yOut)
             const float* skipL = m->skipOut + ((size_t)(L - 1) * B + b) * S;
             for (int s = 0; s < S; s++) skipv[s] = skipL[s];
             float* Zs = m->Zs + (size_t)b * A; float* Za = m->Za + (size_t)b * A; float* P = m->P + (size_t)b * A;
+            const float* skip_q = q16v(m, skipv, S, qs);
             for (int a = 0; a < A; a++) {
-                float v = dot_row(m, m->Wzs, A, S, a, skipv);
+                float v = dot_row(Wzs, A, S, a, skip_q);
                 v = v + q16(m, m->Bzs[a]);
                 v = (v < 0) ? 0.f : v;
                 Zs[a] = v; zs[a] = v;
             }
+            const float* zs_q = q16v(m, zs, A, qz);
             for (int a = 0; a < A; a++) {
-                float v = dot_row(m, m->Wza, A, A, a, zs);
+                float v = dot_row(Wza, A, A, a, zs_q);
                 v = v + q16(m, m->Bza[a]);
                 Za[a] = v;
             }
@@ -337,6 +378,8 @@ int wno_run(wno_model* m, int num_samples, int batch_size, int* yOut)
         }
     }
     free(a_prev); free(a_cur); free(hp); free(h); free(zeroR); free(skipv); free(zs);
+    free(qa); free(qb); free(qh); free(qs); free(qz);
+    for (int i = 0; i < 6; i++) free(wq[i]);
     return status;
 }
 

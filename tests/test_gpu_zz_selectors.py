@@ -5,25 +5,9 @@ import numpy as np
 import pytest
 
 from tests import refgen
+from tests.common import philox_selectors
 
 pytestmark = pytest.mark.gpu
-
-
-def philox_selectors(n, seed):
-    """Host restatement of csrc/wn_convert.cu wn_philox_first: Philox-4x32-10, counter (i, 0), key = seed, first word, 24 bits."""
-    i = np.arange(n, dtype=np.uint64)
-    c0 = (i & np.uint64(0xFFFFFFFF)).astype(np.uint64); c1 = (i >> np.uint64(32)).astype(np.uint64)
-    c2 = np.zeros(n, np.uint64); c3 = np.zeros(n, np.uint64)
-    k0 = np.uint64(seed & 0xFFFFFFFF); k1 = np.uint64((seed >> 32) & 0xFFFFFFFF)
-    M = np.uint64(0xFFFFFFFF)
-    for _ in range(10):
-        p0 = np.uint64(0xD2511F53) * c0
-        p1 = np.uint64(0xCD9E8D57) * c2
-        n0 = ((p1 >> np.uint64(32)) ^ c1 ^ k0) & M; n1 = p1 & M
-        n2 = ((p0 >> np.uint64(32)) ^ c3 ^ k1) & M; n3 = p0 & M
-        c0, c1, c2, c3 = n0, n1, n2, n3
-        k0 = (k0 + np.uint64(0x9E3779B9)) & M; k1 = (k1 + np.uint64(0xBB67AE85)) & M
-    return ((c0 >> np.uint64(8)).astype(np.float32) * np.float32(1.0 / 16777216.0)).astype(np.float32)
 
 
 @pytest.mark.parametrize("dtype_name", ["fp32", "fp16"])
