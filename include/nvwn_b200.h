@@ -35,6 +35,22 @@ enum { NVWN_KERNEL_AUTO = 0, NVWN_KERNEL_STREAM = 16, NVWN_KERNEL_TENSORCORE = 1
 /* nvWavenetInfer::nvWavenetInfer (nv_wavenet.cuh:311) */
 int nvwn_create(nvwn_engine** out, int dtype, int R, int S, int A, int num_layers, int max_dilation,
                 int batch_size, int num_samples, int impl, int tanh_embed);
+/* extension: a WINDOWED engine generates utterances of any length in device memory that does not depend on it.  Same dtypes,
+ * shapes and kernel choice as nvwn_create; `window` (W) replaces num_samples.  Every per-sample store (conditioning, selectors,
+ * yOut) holds W samples and sample t lives in slot t mod W; sample indices run from 0 to 2^31 - 1.  On a windowed engine:
+ *   - nvwn_run_partial takes count <= W; num_samples (the utterance length) only bounds init_sample + count; yOut must be
+ *     NULL (results are read with nvwn_get_yout / nvwn_get_audio).  A run that crosses a multiple of W is two launches.
+ *   - nvwn_set_conditioning, nvwn_cond_producer_run, nvwn_set_conditioning_from_features, nvwn_set_selectors_range and
+ *     nvwn_set_selectors_random_range take absolute sample ranges of at most W samples (a longer one is NVWN_EINVAL).
+ *   - nvwn_get_yout / nvwn_get_audio take an absolute `offset`; the range must lie within the last W samples generated since
+ *     nvwn_reset_history (else NVWN_EINVAL).
+ *   - nvwn_set_inputs, nvwn_set_selectors, nvwn_set_selectors_random and nvwn_set_forced (whole-utterance operations) return
+ *     NVWN_EUNSUPPORTED; there is no teacher forcing.
+ * Writing samples t and t + W reuses one slot: a producer on another stream must wait (cudaStreamWaitEvent) for the run that
+ * consumes t before it overwrites its slot with t + W, and a run must finish before get_yout / get_audio of its samples is
+ * overtaken by the run W samples later -- the same event discipline as nvwn_cond_producer_run. */
+int nvwn_create_windowed(nvwn_engine** out, int dtype, int R, int S, int A, int num_layers, int max_dilation,
+                         int batch_size, int window, int impl, int tanh_embed);
 /* nvWavenetInfer::~nvWavenetInfer (nv_wavenet.cuh:362-395) */
 int nvwn_destroy(nvwn_engine* e);
 const char* nvwn_last_error(void);
@@ -53,6 +69,11 @@ int nvwn_set_conditioning(nvwn_engine* e, const float* Lh, int first_sample, int
  * batch_size + b, is the first output of Philox-4x32-10 with counter (i, 0) and key `seed`, as (x >> 8) * 2^-24 in [0, 1)
  * (the reference draws them on the host with libc rand(), pytorch/wavenet_infer.cu:92-93).  Asynchronous on `stream`. */
 int nvwn_set_selectors_random(nvwn_engine* e, unsigned long long seed, void* stream);
+/* extension, any engine: selectors of samples [first_sample, first_sample + num_samples) only -- from float[num_samples][B]
+ * (host or device; a device source is read in order on `stream`), or drawn on the device with exactly the values
+ * nvwn_set_selectors_random gives those samples (Philox counter sample * batch_size + b). */
+int nvwn_set_selectors_range(nvwn_engine* e, const float* selectors, int first_sample, int num_samples, void* stream);
+int nvwn_set_selectors_random_range(nvwn_engine* e, unsigned long long seed, int first_sample, int num_samples, void* stream);
 /* host helper (needs no GPU): the selectors exactly as the reference wrapper draws them -- Matrix(batch, samples).randomize(0.5, 1.0)
  * on the caller's libc rand() stream (pytorch/wavenet_infer.cu:92-93, matrix.cpp:38-56) -- into selectors[sample * batch_size + b]. */
 int nvwn_libc_selectors(float* selectors, int batch_size, int sample_count);
@@ -94,7 +115,8 @@ int nvwn_weights_updated(nvwn_engine* e);
 int nvwn_run_partial(nvwn_engine* e, int init_sample, int count, int num_samples, int batch_size,
                      int* yOut, int dump_activations, void* stream);
 int nvwn_run(nvwn_engine* e, int num_samples, int batch_size, int* yOut, int dump_activations, void* stream);
-/* nv_wavenet.cuh:439-444: 2-D copy of yOut[b][offset .. offset+size) for every b */
+/* nv_wavenet.cuh:439-444: 2-D copy of yOut[b][offset .. offset+size) for every b.  On a full engine the destination is the
+ * whole int[B][N] array and the samples land at column `offset` (like the reference); on a windowed engine it is int[B][size]. */
 int nvwn_get_yout(nvwn_engine* e, int* yOut, int offset, int size, void* stream);
 /* Output side (SURVEY.md 8f next-3): replaces the host post-processing of pytorch/nv_wavenet_inference.py:55-60 --
  * utils.mu_law_decode_numpy (pytorch/utils.py:62-70) with mu_quantization = A, then MAX_WAV_VALUE * audio and

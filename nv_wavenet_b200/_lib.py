@@ -23,6 +23,7 @@ class LaunchInfo(C.Structure):
 # every symbol include/*.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "nvwn_create": (C.c_int, [C.POINTER(_vp)] + [C.c_int] * 10),
+    "nvwn_create_windowed": (C.c_int, [C.POINTER(_vp)] + [C.c_int] * 10),
     "nvwn_destroy": (C.c_int, [_vp]),
     "nvwn_last_error": (C.c_char_p, []),
     "nvwn_set_embeddings": (C.c_int, [_vp, _vp, _vp]),
@@ -32,6 +33,8 @@ SYMBOLS = {
     "nvwn_set_selectors": (C.c_int, [_vp, _vp]),
     "nvwn_set_conditioning": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp]),
     "nvwn_set_selectors_random": (C.c_int, [_vp, C.c_ulonglong, _vp]),
+    "nvwn_set_selectors_range": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp]),
+    "nvwn_set_selectors_random_range": (C.c_int, [_vp, C.c_ulonglong, C.c_int, C.c_int, _vp]),
     "nvwn_libc_selectors": (C.c_int, [_vp, C.c_int, C.c_int]),
     "nvwn_reset_history": (C.c_int, [_vp]),
     "nvwn_set_forced": (C.c_int, [_vp, _vp]),

@@ -10,8 +10,11 @@
 struct WnParams {
     int L, R, S, A, maxDil;
     int B;              // batch size of this run (stride of Lh / selectors / ring, nv_wavenet.cuh:144)
-    int N;              // num_samples of this run (row stride of yOut, singleblock.cuh:245)
+    int N;              // row stride of yOut: num_samples of this run (singleblock.cuh:245), the window W on windowed engines
     int init_sample, count;
+    // window origin: the absolute sample held in slot 0 of every per-sample store (Lh, sel, forced, yOut); sample t lives in slot
+    // t - origin.  0 on full engines.  The sample index t itself stays absolute (dilation mask, history-ring slot).
+    int origin;
     int tanhEmbed, dump;
     // model (TD = float in fp32 mode, __half in fp16 mode)
     const void *embPrev, *embCur;                       // TD [A][R]
@@ -44,5 +47,5 @@ bool wn_stream_supported(int R, int S, int A, bool fp16);
 // conversions (wn_convert.cu)
 cudaError_t wn_f32_to_f16(__half* dst, const float* src_dev, size_t n, cudaStream_t stream);
 cudaError_t wn_f16_to_f32(float* dst, const __half* src_dev, size_t n, cudaStream_t stream);
-cudaError_t wn_fill_selectors(float* dst, size_t n, unsigned long long seed, cudaStream_t stream);
+cudaError_t wn_fill_selectors(float* dst, size_t n, unsigned long long first, unsigned long long seed, cudaStream_t stream);   // counters first..first+n-1
 cudaError_t wn_fill_int(int* dst, int value, size_t n, cudaStream_t stream);

@@ -18,16 +18,17 @@ __global__ void f32_to_f16_kernel(__half* __restrict__ dst, const float* __restr
     }
     for (size_t j = n4 * 4 + i; j < n; j += stride) dst[j] = __float2half_rn(src[j]);
 }
-// mu-law decode of sampled indices, table-driven: out[b][j] = lut[yOut[b * N + offset + j]]
-__global__ void mulaw_decode_kernel(const int* __restrict__ y, int N, int offset, int size, size_t total, int A, const float* __restrict__ lut_f,
-                                    const short* __restrict__ lut_s, float* __restrict__ out_f, short* __restrict__ out_s)
+// mu-law decode of sampled indices, table-driven: out[b * out_pitch + j] = lut[yOut[b * N + offset + j]]
+__global__ void mulaw_decode_kernel(const int* __restrict__ y, int N, int offset, int size, size_t out_pitch, size_t total, int A,
+                                    const float* __restrict__ lut_f, const short* __restrict__ lut_s, float* __restrict__ out_f,
+                                    short* __restrict__ out_s)
 {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-        const size_t b = i / (size_t)size, j = i % (size_t)size;
+        const size_t b = i / (size_t)size, j = i % (size_t)size, o = b * out_pitch + j;
         int v = y[b * (size_t)N + offset + j];
         v = v < 0 ? 0 : (v >= A ? A - 1 : v);
-        if (out_f) out_f[i] = lut_f[v];
-        if (out_s) out_s[i] = lut_s[v];
+        if (out_f) out_f[o] = lut_f[v];
+        if (out_s) out_s[o] = lut_s[v];
     }
 }
 __global__ void fill_int_kernel(int* dst, int v, size_t n)
@@ -63,6 +64,7 @@ cudaError_t wn_f16_to_f32(float* dst, const __half* src_dev, size_t n, cudaStrea
 // Counter-based selectors (SURVEY.md 8f next-1: "device-side Philox selectors"): element i of the [N][B] selector array is the
 // first 32-bit output of Philox-4x32-10 with counter (i_lo, i_hi, 0, 0) and key (seed_lo, seed_hi), mapped to [0, 1) with
 // 24 bits: (x >> 8) * 2^-24.  Stateless, order-independent, reproducible on the host (tests/test_gpu_zz_selectors.py).
+// dst[i] takes counter first + i, so a range of samples can be drawn on its own: first = first_sample * B.
 __host__ __device__ inline unsigned wn_philox_first(unsigned long long ctr, unsigned long long seed)
 {
     unsigned c0 = (unsigned)ctr, c1 = (unsigned)(ctr >> 32), c2 = 0, c3 = 0;
@@ -75,17 +77,17 @@ __host__ __device__ inline unsigned wn_philox_first(unsigned long long ctr, unsi
     }
     return c0;
 }
-__global__ void selectors_kernel(float* __restrict__ dst, size_t n, unsigned long long seed)
+__global__ void selectors_kernel(float* __restrict__ dst, size_t n, unsigned long long first, unsigned long long seed)
 {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
-        dst[i] = (float)(wn_philox_first(i, seed) >> 8) * (1.0f / 16777216.0f);
+        dst[i] = (float)(wn_philox_first(first + i, seed) >> 8) * (1.0f / 16777216.0f);
 }
-cudaError_t wn_fill_selectors(float* dst, size_t n, unsigned long long seed, cudaStream_t stream)
+cudaError_t wn_fill_selectors(float* dst, size_t n, unsigned long long first, unsigned long long seed, cudaStream_t stream)
 {
     if (n == 0) return cudaSuccess;
     size_t blocks = (n + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;
-    selectors_kernel<<<(unsigned)blocks, 256, 0, stream>>>(dst, n, seed);
+    selectors_kernel<<<(unsigned)blocks, 256, 0, stream>>>(dst, n, first, seed);
     return cudaGetLastError();
 }
 
@@ -99,12 +101,12 @@ cudaError_t wn_fill_int(int* dst, int value, size_t n, cudaStream_t stream)
 }
 
 cudaError_t wn_mulaw_decode(const int* yOut, int N, int offset, int size, int B, int A, const float* lut_f, const short* lut_s, float* out_f,
-                            short* out_s, cudaStream_t stream)
+                            short* out_s, size_t out_pitch, cudaStream_t stream)
 {
     const size_t total = (size_t)B * size;
     if (total == 0) return cudaSuccess;
     size_t blocks = (total + 255) / 256;
     if (blocks > 148 * 8) blocks = 148 * 8;
-    mulaw_decode_kernel<<<(unsigned)blocks, 256, 0, stream>>>(yOut, N, offset, size, total, A, lut_f, lut_s, out_f, out_s);
+    mulaw_decode_kernel<<<(unsigned)blocks, 256, 0, stream>>>(yOut, N, offset, size, out_pitch, total, A, lut_f, lut_s, out_f, out_s);
     return cudaGetLastError();
 }

@@ -10,6 +10,7 @@
 #include "../../include/nvwn_b200.h"
 #include "wn_common.h"
 
+#include <limits.h>
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -26,7 +27,7 @@ cudaError_t wn_cond_produce(float* out, float* U, const float* feat, const float
 void wn_cond_host(float* Lh, const float* feat, const float* Wu, const float* bu, const float* Wc, const float* bc,
                   int B, int C, int T, int K, int stride, int L, int R);
 cudaError_t wn_mulaw_decode(const int* yOut, int N, int offset, int size, int B, int A, const float* lut_f, const short* lut_s, float* out_f,
-                            short* out_s, cudaStream_t stream);                                                  // wn_convert.cu
+                            short* out_s, size_t out_pitch, cudaStream_t stream);                                // wn_convert.cu
 size_t wn_tc_image_bytes(int R, int S, int A, int L);
 cudaError_t wn_tc_pack(void* image, const WnParams& p, cudaStream_t stream);
 size_t wn_tc_ring_bytes(int TU, int L, int maxDil, int B);
@@ -75,6 +76,9 @@ bool is_device_ptr(const void* p)
 struct nvwn_engine {
     int dtype, R, S, A, L, maxDil, B, N, impl, tanhEmbed, device;
     size_t td;                               // sizeof(TD)
+    // windowed engine (nvwn_create_windowed): every per-sample store holds N = W samples, sample t in slot t % W; 0 = full engine
+    int W = 0;
+    long long gen_lo = 0, gen_hi = -1;       // windowed: samples [gen_lo, gen_hi) generated back to back since nvwn_reset_history
 
     // packed weight blob (TD elements), offsets in bytes
     char* blob = nullptr;
@@ -83,7 +87,7 @@ struct nvwn_engine {
 
     void* Lh = nullptr;                      // TD [N][L][B][2R]
     float* sel = nullptr;                    // [N][B]
-    int* forced = nullptr;                   // [B][N]
+    int* forced = nullptr;                   // [B][N]; not allocated on windowed engines
     bool use_forced = false;
     int *yPrev = nullptr, *yCur = nullptr, *yOut = nullptr;
     void* ring = nullptr;
@@ -169,11 +173,12 @@ int decide_fp16_kernel(int dtype, int impl, int R, int S, int A, int L, int B)
     return tc_ok ? 1 : 0;
 }
 
-void fill_params(const nvwn_engine* e, WnParams& p, int init_sample, int count, int num_samples, int batch, int dump)
+// `pitch` = yOut row stride (num_samples, or W on windowed engines); `origin` = the absolute sample held in slot 0 of the stores
+void fill_params(const nvwn_engine* e, WnParams& p, int init_sample, int count, int pitch, int origin, int batch, int dump)
 {
     memset(&p, 0, sizeof p);
     p.L = e->L; p.R = e->R; p.S = e->S; p.A = e->A; p.maxDil = e->maxDil;
-    p.B = batch; p.N = num_samples; p.init_sample = init_sample; p.count = count;
+    p.B = batch; p.N = pitch; p.init_sample = init_sample; p.count = count; p.origin = origin;
     p.tanhEmbed = e->tanhEmbed; p.dump = dump;
     p.embPrev = e->blob + e->o_embPrev; p.embCur = e->blob + e->o_embCur;
     p.Wprev = e->blob + e->o_Wprev; p.Wcur = e->blob + e->o_Wcur; p.Wres = e->blob + e->o_Wres; p.Wskip = e->blob + e->o_Wskip;
@@ -184,6 +189,54 @@ void fill_params(const nvwn_engine* e, WnParams& p, int init_sample, int count, 
     p.xtOut = e->xtOut; p.skipOut = e->skipOut; p.Zs = e->Zs; p.Za = e->Za; p.P = e->P;
     p.trace = e->trace; p.trace_t = e->trace_t;
 }
+
+// Splits the absolute sample range [first, first + n) of a windowed engine's store at multiples of W: f(slot, offset into the
+// range, length) per piece (one piece, or two where the range crosses the window edge).  On a full engine slot = first.
+template <typename F>
+int for_slots(const nvwn_engine* e, long long first, long long n, F f)
+{
+    if (!e->W) return n > 0 ? f((int)first, 0, (int)n) : 0;
+    for (long long done = 0; done < n;) {
+        const int slot = (int)((first + done) % e->W);
+        const long long m = (n - done < e->W - slot) ? n - done : e->W - slot;
+        const int rc = f(slot, (int)done, (int)m);
+        if (rc) return rc;
+        done += m;
+    }
+    return 0;
+}
+
+// the range check of the absolute-sample setters: a full engine holds [0, N); a windowed one takes any range of at most W samples
+// with indices below 2^31
+int check_range(const nvwn_engine* e, const char* fn, long long first, long long n)
+{
+    if (first < 0 || n < 0) return fail(NVWN_EINVAL, std::string(fn) + ": sample range out of bounds");
+    if (!e->W) return first + n > e->N ? fail(NVWN_EINVAL, std::string(fn) + ": sample range out of bounds") : 0;
+    if (n > e->W) return fail(NVWN_EINVAL, std::string(fn) + ": " + std::to_string(n) + " samples exceed the window of " + std::to_string(e->W));
+    if (first + n > INT_MAX) return fail(NVWN_EINVAL, std::string(fn) + ": sample indices end at 2^31 - 1");
+    return 0;
+}
+
+// the output getters of a windowed engine: the range must lie within the last W samples generated since nvwn_reset_history
+int check_window_read(const nvwn_engine* e, const char* fn, long long offset, long long size)
+{
+    const long long lo = e->gen_hi - e->W > e->gen_lo ? e->gen_hi - e->W : e->gen_lo;
+    if (offset < 0 || size < 0 || (size > 0 && (offset < lo || offset + size > e->gen_hi)))
+        return fail(NVWN_EINVAL, std::string(fn) + ": samples [" + std::to_string(offset) + ", " + std::to_string(offset + size) +
+                                     ") are not within the last window of generated samples [" + std::to_string(lo) + ", " +
+                                     std::to_string(e->gen_hi < 0 ? 0 : e->gen_hi) + ")");
+    return 0;
+}
+
+int windowed_unsupported(const nvwn_engine* e, const char* fn)
+{
+    return fail(NVWN_EUNSUPPORTED, std::string(fn) + ": a windowed engine (window " + std::to_string(e->W) +
+                                       ") has no whole-utterance stores; use the range setters (nvwn_set_conditioning, "
+                                       "nvwn_set_selectors_range, nvwn_set_selectors_random_range)");
+}
+
+int create_engine(nvwn_engine** out, const char* fn, int dtype, int R, int S, int A, int num_layers, int max_dilation,
+                  int batch_size, int num_samples, int window, int impl, int tanh_embed);
 
 }  // namespace
 
@@ -207,20 +260,38 @@ int nvwn_set_device(int device)
 int nvwn_create(nvwn_engine** out, int dtype, int R, int S, int A, int num_layers, int max_dilation,
                 int batch_size, int num_samples, int impl, int tanh_embed)
 {
-    if (!out) return fail(NVWN_EINVAL, "nvwn_create: out is NULL");
+    return create_engine(out, "nvwn_create", dtype, R, S, A, num_layers, max_dilation, batch_size, num_samples, 0, impl, tanh_embed);
+}
+
+int nvwn_create_windowed(nvwn_engine** out, int dtype, int R, int S, int A, int num_layers, int max_dilation,
+                         int batch_size, int window, int impl, int tanh_embed)
+{
+    return create_engine(out, "nvwn_create_windowed", dtype, R, S, A, num_layers, max_dilation, batch_size, window, window, impl, tanh_embed);
+}
+
+}  // extern "C"
+
+namespace {
+
+// num_samples = the length of every per-sample store: N of a full engine, W (= window) of a windowed one
+int create_engine(nvwn_engine** out, const char* fn, int dtype, int R, int S, int A, int num_layers, int max_dilation,
+                  int batch_size, int num_samples, int window, int impl, int tanh_embed)
+{
+    const std::string f(fn);
+    if (!out) return fail(NVWN_EINVAL, f + ": out is NULL");
     *out = nullptr;
-    if (dtype != NVWN_FP32 && dtype != NVWN_FP16 && dtype != NVWN_FP32_FAST) return fail(NVWN_EINVAL, "nvwn_create: dtype must be NVWN_FP32, NVWN_FP16 or NVWN_FP32_FAST");
-    if (num_layers < 1 || max_dilation < 1 || batch_size < 1 || num_samples < 1) return fail(NVWN_EINVAL, "nvwn_create: sizes must be positive");
+    if (dtype != NVWN_FP32 && dtype != NVWN_FP16 && dtype != NVWN_FP32_FAST) return fail(NVWN_EINVAL, f + ": dtype must be NVWN_FP32, NVWN_FP16 or NVWN_FP32_FAST");
+    if (num_layers < 1 || max_dilation < 1 || batch_size < 1 || num_samples < 1) return fail(NVWN_EINVAL, f + ": sizes must be positive");
     if (!wn_stream_supported(R, S, A, dtype == NVWN_FP16))
-        return fail(NVWN_EUNSUPPORTED, "nvwn_create: unsupported channel counts (R,S) must be one of (32,128) (64,128) (64,256) (128,256); A a multiple of 32");
+        return fail(NVWN_EUNSUPPORTED, f + ": unsupported channel counts (R,S) must be one of (32,128) (64,128) (64,256) (128,256); A a multiple of 32");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
         cudaGetLastError();
-        return fail(NVWN_EUNSUPPORTED, "nvwn_create: no CUDA device (this engine has no CPU fallback)");
+        return fail(NVWN_EUNSUPPORTED, f + ": no CUDA device (this engine has no CPU fallback)");
     }
     nvwn_engine* e = new nvwn_engine();
     e->dtype = dtype; e->R = R; e->S = S; e->A = A; e->L = num_layers; e->maxDil = max_dilation;
-    e->B = batch_size; e->N = num_samples; e->impl = impl; e->tanhEmbed = tanh_embed ? 1 : 0;
+    e->B = batch_size; e->N = num_samples; e->W = window; e->impl = impl; e->tanhEmbed = tanh_embed ? 1 : 0;
     e->td = dtype == NVWN_FP16 ? 2 : 4;
     cudaGetDevice(&e->device);
 
@@ -256,7 +327,7 @@ int nvwn_create(nvwn_engine** out, int dtype, int R, int S, int A, int num_layer
     ALLOC(e->Lh, e->tc_mode ? wn_tc_cond_bytes(e->tc_tile, num_layers, batch_size, num_samples)
                  : e->lat_mode ? wn_lat_cond_bytes(num_layers, batch_size, num_samples) : Nz * L * Bz * 2 * R * td);
     ALLOC(e->sel, Nz * Bz * sizeof(float));
-    ALLOC(e->forced, Nz * Bz * sizeof(int));
+    if (!window) ALLOC(e->forced, Nz * Bz * sizeof(int));           // teacher forcing is a whole-utterance operation
     ALLOC(e->yPrev, Bz * sizeof(int));
     ALLOC(e->yCur, Bz * sizeof(int));
     ALLOC(e->yOut, Nz * Bz * sizeof(int));
@@ -286,6 +357,10 @@ int nvwn_create(nvwn_engine** out, int dtype, int R, int S, int A, int num_layer
     *out = e;
     return 0;
 }
+
+}  // namespace
+
+extern "C" {
 
 int nvwn_destroy(nvwn_engine* e)
 {
@@ -389,7 +464,9 @@ int nvwn_cond_producer_run(nvwn_engine* e, int first_sample, int sample_begin, i
     const int C = e->cp_C, T = e->cp_T, K = e->cp_K, stride = e->cp_stride, chunk = e->cp_chunk;
     const long long Nn = (long long)T * stride;
     if (sample_begin < 0 || sample_count < 0 || sample_begin + (long long)sample_count > Nn) return fail(NVWN_EINVAL, "nvwn_cond_producer_run: sample range outside num_frames * stride");
-    if (first_sample < 0 || first_sample + (long long)sample_begin + sample_count > e->N) return fail(NVWN_EINVAL, "nvwn_cond_producer_run: samples do not fit the engine");
+    if (e->W) {
+        if (int rc = check_range(e, "nvwn_cond_producer_run", (long long)first_sample + sample_begin, sample_count)) return rc;
+    } else if (first_sample < 0 || first_sample + (long long)sample_begin + sample_count > e->N) return fail(NVWN_EINVAL, "nvwn_cond_producer_run: samples do not fit the engine");
     cudaStream_t st = (cudaStream_t)stream;
     const size_t per = (size_t)e->L * e->B * 2 * e->R;
     const size_t n_feat = (size_t)e->B * C * T, n_wu = (size_t)C * C * K, n_wc = (size_t)e->L * 2 * e->R * C, n_bc = (size_t)e->L * 2 * e->R;
@@ -415,7 +492,9 @@ int nvwn_set_conditioning_from_features(nvwn_engine* e, const float* features, i
 {
     if (!e) return fail(NVWN_EINVAL, "nvwn_set_conditioning_from_features: NULL argument");
     const long long Nn = (long long)num_frames * stride;
-    if (first_sample < 0 || (num_frames >= 1 && stride >= 1 && first_sample + Nn > e->N)) return fail(NVWN_EINVAL, "nvwn_set_conditioning_from_features: num_frames * stride samples do not fit the engine");
+    if (e->W && num_frames >= 1 && stride >= 1) {
+        if (int rc = check_range(e, "nvwn_set_conditioning_from_features", first_sample, Nn)) return rc;
+    } else if (first_sample < 0 || (num_frames >= 1 && stride >= 1 && first_sample + Nn > e->N)) return fail(NVWN_EINVAL, "nvwn_set_conditioning_from_features: num_frames * stride samples do not fit the engine");
     int rc = nvwn_cond_producer_load(e, features, n_cond_channels, num_frames, upsample_weight, upsample_bias, window, stride, cond_weight, cond_bias, stream);
     if (rc != 0) return rc;
     rc = nvwn_cond_producer_run(e, first_sample, 0, (int)Nn, stream);
@@ -427,6 +506,7 @@ int nvwn_set_conditioning_from_features(nvwn_engine* e, const float* features, i
 int nvwn_reset_history(nvwn_engine* e)
 {
     if (!e) return fail(NVWN_EINVAL, "nvwn_reset_history: NULL engine");
+    e->gen_lo = 0; e->gen_hi = -1;
     CK(wn_fill_int(e->yPrev, 128, e->B, 0));      // silenceInputs, nv_wavenet.cuh:213-218
     CK(wn_fill_int(e->yCur, 128, e->B, 0));
     return 0;
@@ -435,6 +515,7 @@ int nvwn_reset_history(nvwn_engine* e)
 int nvwn_set_selectors(nvwn_engine* e, const float* selectors)
 {
     if (!e || !selectors) return fail(NVWN_EINVAL, "nvwn_set_selectors: NULL argument");
+    if (e->W) return windowed_unsupported(e, "nvwn_set_selectors");
     CK(cudaMemcpy(e->sel, selectors, (size_t)e->N * e->B * sizeof(float), cudaMemcpyDefault));
     return 0;
 }
@@ -459,14 +540,42 @@ int nvwn_libc_selectors(float* selectors, int batch_size, int sample_count)
 int nvwn_set_selectors_random(nvwn_engine* e, unsigned long long seed, void* stream)
 {
     if (!e) return fail(NVWN_EINVAL, "nvwn_set_selectors_random: NULL engine");
-    CK(wn_fill_selectors(e->sel, (size_t)e->N * e->B, seed, (cudaStream_t)stream));
+    if (e->W) return windowed_unsupported(e, "nvwn_set_selectors_random");
+    CK(wn_fill_selectors(e->sel, (size_t)e->N * e->B, 0, seed, (cudaStream_t)stream));
     return 0;
 }
 
-int nvwn_set_conditioning(nvwn_engine* e, const float* Lh, int first_sample, int num_samples, void* stream)
+int nvwn_set_selectors_range(nvwn_engine* e, const float* selectors, int first_sample, int num_samples, void* stream)
 {
-    if (!e || !Lh) return fail(NVWN_EINVAL, "nvwn_set_conditioning: NULL argument");
-    if (first_sample < 0 || num_samples < 0 || first_sample + num_samples > e->N) return fail(NVWN_EINVAL, "nvwn_set_conditioning: sample range out of bounds");
+    if (!e || !selectors) return fail(NVWN_EINVAL, "nvwn_set_selectors_range: NULL argument");
+    if (int rc = check_range(e, "nvwn_set_selectors_range", first_sample, num_samples)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t B = e->B;
+    int rc = for_slots(e, first_sample, num_samples, [&](int slot, int done, int m) {
+        CK(cudaMemcpyAsync(e->sel + (size_t)slot * B, selectors + (size_t)done * B, (size_t)m * B * sizeof(float), cudaMemcpyDefault, st));
+        return 0;
+    });
+    if (rc) return rc;
+    if (!is_device_ptr(selectors)) CK(cudaStreamSynchronize(st));      // host source: copied before return
+    return 0;
+}
+
+int nvwn_set_selectors_random_range(nvwn_engine* e, unsigned long long seed, int first_sample, int num_samples, void* stream)
+{
+    if (!e) return fail(NVWN_EINVAL, "nvwn_set_selectors_random_range: NULL engine");
+    if (int rc = check_range(e, "nvwn_set_selectors_random_range", first_sample, num_samples)) return rc;
+    const size_t B = e->B;
+    return for_slots(e, first_sample, num_samples, [&](int slot, int done, int m) {
+        CK(wn_fill_selectors(e->sel + (size_t)slot * B, (size_t)m * B, ((unsigned long long)first_sample + done) * B, seed, (cudaStream_t)stream));
+        return 0;
+    });
+}
+
+namespace {
+
+// conditioning of store slots [first_sample, first_sample + num_samples) <- Lh (fp32 [num_samples][L][B][2R], host or device)
+int put_conditioning(nvwn_engine* e, const float* Lh, int first_sample, int num_samples, void* stream)
+{
     const size_t per = (size_t)e->L * e->B * 2 * e->R;
     if (!e->tc_mode && !e->lat_mode)
         return upload(e, static_cast<char*>(e->Lh) + (size_t)first_sample * per * e->td, Lh, per * num_samples, (cudaStream_t)stream);
@@ -492,9 +601,22 @@ int nvwn_set_conditioning(nvwn_engine* e, const float* Lh, int first_sample, int
     return 0;
 }
 
+}  // namespace
+
+int nvwn_set_conditioning(nvwn_engine* e, const float* Lh, int first_sample, int num_samples, void* stream)
+{
+    if (!e || !Lh) return fail(NVWN_EINVAL, "nvwn_set_conditioning: NULL argument");
+    if (int rc = check_range(e, "nvwn_set_conditioning", first_sample, num_samples)) return rc;
+    const size_t per = (size_t)e->L * e->B * 2 * e->R;
+    return for_slots(e, first_sample, num_samples, [&](int slot, int done, int m) {
+        return put_conditioning(e, Lh + (size_t)done * per, slot, m, stream);
+    });
+}
+
 int nvwn_set_inputs(nvwn_engine* e, const float* Lh, const float* selectors)
 {
     if (!e || !Lh || !selectors) return fail(NVWN_EINVAL, "nvwn_set_inputs: NULL argument");
+    if (e->W) return windowed_unsupported(e, "nvwn_set_inputs");
     int rc;
     if ((rc = nvwn_reset_history(e))) return rc;
     if ((rc = nvwn_set_conditioning(e, Lh, 0, e->N, nullptr))) return rc;
@@ -506,6 +628,7 @@ int nvwn_set_inputs(nvwn_engine* e, const float* Lh, const float* selectors)
 int nvwn_set_forced(nvwn_engine* e, const int* forced)
 {
     if (!e) return fail(NVWN_EINVAL, "nvwn_set_forced: NULL engine");
+    if (e->W) return windowed_unsupported(e, "nvwn_set_forced");
     if (!forced) { e->use_forced = false; return 0; }
     CK(cudaMemcpy(e->forced, forced, (size_t)e->N * e->B * sizeof(int), cudaMemcpyDefault));
     e->use_forced = true;
@@ -527,39 +650,67 @@ int nvwn_weights_updated(nvwn_engine* e)
     return 0;
 }
 
+namespace {
+
+// one kernel launch over samples [p.init_sample, p.init_sample + p.count), all in one window period of the stores
+int launch(nvwn_engine* e, const WnParams& p, int batch_size, cudaStream_t stream)
+{
+    if (e->lat_mode) {
+        // a smaller batch_size runs the first batch_size utterances of the engine's batch (conditioning was laid out per
+        // 16-utterance tile for the engine's batch size at upload)
+        if (e->tc_dirty) {
+            CK(wn_lat_pack(e->tc_image, p, stream));
+            e->tc_dirty = false;
+        }
+        CK(wn_launch_lat(p, e->tc_image, e->B, e->lat_cluster, stream, &e->last));
+    } else if (e->tc_mode) {
+        if (batch_size != e->B)
+            return fail(NVWN_EINVAL, "nvwn_run_partial: the tensor-core path needs batch_size equal to the engine's batch size");
+        if (e->tc_dirty) {
+            CK(wn_tc_pack(e->tc_image, p, stream));
+            e->tc_dirty = false;
+        }
+        CK(wn_launch_tc(p, e->tc_image, e->tc_tile, e->tc_fused, stream, &e->last));
+    } else {
+        CK(wn_launch_stream(p, e->dtype == NVWN_FP16 ? 1 : (e->dtype == NVWN_FP32_FAST ? 2 : 0), stream, &e->last));
+    }
+    e->launches++;
+    return 0;
+}
+
+}  // namespace
+
 int nvwn_run_partial(nvwn_engine* e, int init_sample, int count, int num_samples, int batch_size,
                      int* yOut, int dump_activations, void* stream_)
 {
     if (!e) return fail(NVWN_EINVAL, "nvwn_run_partial: NULL engine");
-    if (batch_size < 1 || batch_size > e->B || num_samples < 1 || num_samples > e->N)
+    if (batch_size < 1 || batch_size > e->B || num_samples < 1 || (!e->W && num_samples > e->N))
         return fail(NVWN_EINVAL, "nvwn_run_partial: batch_size / num_samples exceed what the engine was created for");
-    if (init_sample < 0 || count < 0 || init_sample + count > num_samples) return fail(NVWN_EINVAL, "nvwn_run_partial: sample range out of bounds");
+    if (init_sample < 0 || count < 0 || (long long)init_sample + count > num_samples) return fail(NVWN_EINVAL, "nvwn_run_partial: sample range out of bounds");
     cudaStream_t stream = (cudaStream_t)stream_;
+    const int dump = dump_activations ? 1 : 0;
     WnParams p;
-    fill_params(e, p, init_sample, count, num_samples, batch_size, dump_activations ? 1 : 0);
-    if (count > 0) {
-        if (e->lat_mode) {
-            // a smaller batch_size runs the first batch_size utterances of the engine's batch (conditioning was laid out per
-            // 16-utterance tile for the engine's batch size at upload)
-            if (e->tc_dirty) {
-                CK(wn_lat_pack(e->tc_image, p, stream));
-                e->tc_dirty = false;
-            }
-            CK(wn_launch_lat(p, e->tc_image, e->B, e->lat_cluster, stream, &e->last));
-        } else if (e->tc_mode) {
-            if (batch_size != e->B)
-                return fail(NVWN_EINVAL, "nvwn_run_partial: the tensor-core path needs batch_size equal to the engine's batch size");
-            if (e->tc_dirty) {
-                CK(wn_tc_pack(e->tc_image, p, stream));
-                e->tc_dirty = false;
-            }
-            CK(wn_launch_tc(p, e->tc_image, e->tc_tile, e->tc_fused, stream, &e->last));
-        } else {
-            CK(wn_launch_stream(p, e->dtype == NVWN_FP16 ? 1 : (e->dtype == NVWN_FP32_FAST ? 2 : 0), stream, &e->last));
-        }
-        e->launches++;
+    if (!e->W) {
+        fill_params(e, p, init_sample, count, num_samples, 0, batch_size, dump);
+        if (count > 0)
+            if (int rc = launch(e, p, batch_size, stream)) return rc;
+        if (yOut) CK(cudaMemcpyAsync(yOut, e->yOut, (size_t)num_samples * batch_size * sizeof(int), cudaMemcpyDefault, stream));
+        return 0;
     }
-    if (yOut) CK(cudaMemcpyAsync(yOut, e->yOut, (size_t)num_samples * batch_size * sizeof(int), cudaMemcpyDefault, stream));
+    // windowed: the stores hold samples [k W, (k + 1) W) at a time, so a run that crosses a multiple of W is two launches (the
+    // history ring and the feedback indices carry over between them exactly as between any two run_partial calls)
+    if (yOut) return fail(NVWN_EINVAL, "nvwn_run_partial: yOut must be NULL on a windowed engine (read results with nvwn_get_yout / nvwn_get_audio)");
+    if (count > e->W) return fail(NVWN_EINVAL, "nvwn_run_partial: count " + std::to_string(count) + " exceeds the window of " + std::to_string(e->W));
+    int rc = for_slots(e, init_sample, count, [&](int slot, int done, int m) {
+        const int t0 = init_sample + done;
+        fill_params(e, p, t0, m, e->W, t0 - slot, batch_size, dump && done + m == count);
+        return launch(e, p, batch_size, stream);
+    });
+    if (rc) return rc;
+    if (count > 0) {
+        if (init_sample != e->gen_hi) e->gen_lo = init_sample;
+        e->gen_hi = (long long)init_sample + count;
+    }
     return 0;
 }
 
@@ -571,6 +722,14 @@ int nvwn_run(nvwn_engine* e, int num_samples, int batch_size, int* yOut, int dum
 int nvwn_get_yout(nvwn_engine* e, int* yOut, int offset, int size, void* stream)
 {
     if (!e || !yOut) return fail(NVWN_EINVAL, "nvwn_get_yout: NULL argument");
+    if (e->W) {                                   // destination [B][size]; source rows of W slots, split at the window edge
+        if (int rc = check_window_read(e, "nvwn_get_yout", offset, size)) return rc;
+        return for_slots(e, offset, size, [&](int slot, int done, int m) {
+            CK(cudaMemcpy2DAsync(yOut + done, (size_t)size * sizeof(int), e->yOut + slot, (size_t)e->W * sizeof(int), (size_t)m * sizeof(int),
+                                 e->B, cudaMemcpyDefault, (cudaStream_t)stream));
+            return 0;
+        });
+    }
     if (offset < 0 || size < 0 || offset + size > e->N) return fail(NVWN_EINVAL, "nvwn_get_yout: range out of bounds");
     if (size == 0) return 0;
     const size_t pitch = (size_t)e->N * sizeof(int);
@@ -619,7 +778,9 @@ int nvwn_mulaw_table(int A, float* f32, short* i16_wrap, short* i16_saturate)
 int nvwn_get_audio(nvwn_engine* e, float* audio_f32, short* audio_i16, int offset, int size, int saturate, void* stream)
 {
     if (!e || (!audio_f32 && !audio_i16)) return fail(NVWN_EINVAL, "nvwn_get_audio: NULL argument");
-    if (offset < 0 || size < 0 || offset + size > e->N) return fail(NVWN_EINVAL, "nvwn_get_audio: range out of bounds");
+    if (e->W) {
+        if (int rc = check_window_read(e, "nvwn_get_audio", offset, size)) return rc;
+    } else if (offset < 0 || size < 0 || offset + size > e->N) return fail(NVWN_EINVAL, "nvwn_get_audio: range out of bounds");
     if (size == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     const int A = e->A;
@@ -643,7 +804,11 @@ int nvwn_get_audio(nvwn_engine* e, float* audio_f32, short* audio_i16, int offse
         if (!f_dev) df = static_cast<float*>(tmp);
         if (!s_dev) ds = reinterpret_cast<short*>(static_cast<char*>(tmp) + total * sizeof(float));
     }
-    cudaError_t ce = wn_mulaw_decode(e->yOut, e->N, offset, size, e->B, A, e->lut_f, lut_s, df, ds, st);
+    cudaError_t ce = cudaSuccess;
+    for_slots(e, offset, size, [&](int slot, int done, int m) {       // windowed: split at the window edge
+        if (ce == cudaSuccess) ce = wn_mulaw_decode(e->yOut, e->N, slot, m, e->B, A, e->lut_f, lut_s, df ? df + done : nullptr, ds ? ds + done : nullptr, (size_t)size, st);
+        return 0;
+    });
     if (ce == cudaSuccess && !f_dev) ce = cudaMemcpyAsync(audio_f32, df, total * sizeof(float), cudaMemcpyDeviceToHost, st);
     if (ce == cudaSuccess && !s_dev) ce = cudaMemcpyAsync(audio_i16, ds, total * sizeof(short), cudaMemcpyDeviceToHost, st);
     if (tmp) {

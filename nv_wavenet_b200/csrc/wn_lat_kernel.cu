@@ -470,7 +470,7 @@ __global__ void __launch_bounds__(NT, 1) wn_lat_kernel(const WnParams p, const u
         float sk[C::NSK][4];
 #pragma unroll
         for (int i = 0; i < C::NSK; i++) sk[i][0] = sk[i][1] = sk[i][2] = sk[i][3] = 0.f;
-        const unsigned char* cptr = gcond + (size_t)t_begin * L * cstride;      // conditioning of step it3 (steps are consecutive in memory)
+        const unsigned char* cptr = gcond + (size_t)(t_begin - p.origin) * L * cstride;      // conditioning of step it3 (steps are consecutive in memory)
 
         // accp <- (Bh + Lh) + Wprev . x[t-d] for the coming step `it1` (its staged history tile is number `pn`, its conditioning
         // sits in cbA / cbB by parity); Wprev rides in the SAME ring piece as the current layer's Wcur (`p1`; the very first
@@ -637,8 +637,8 @@ __global__ void __launch_bounds__(NT, 1) wn_lat_kernel(const WnParams p, const u
         for (int t = t_begin; t < t_end; t++) {
             // ---------------- embedding (reference.cpp:42-57): x0 = [tanh](embPrev[yPrev] + embCur[yCur]), this warp's 8 channels
             if (tid == 0) TRACE(0, 1);
-            const float sel0 = (2 * w + 0 + tile * TU) < B ? p.sel[(size_t)t * B + tile * TU + 2 * w] : 0.5f;
-            const float sel1 = (2 * w + 1 + tile * TU) < B ? p.sel[(size_t)t * B + tile * TU + 2 * w + 1] : 0.5f;
+            const float sel0 = (2 * w + 0 + tile * TU) < B ? p.sel[(size_t)(t - p.origin) * B +tile * TU + 2 * w] : 0.5f;
+            const float sel1 = (2 * w + 1 + tile * TU) < B ? p.sel[(size_t)(t - p.origin) * B +tile * TU + 2 * w + 1] : 0.5f;
             {
                 const int yc0 = ys[g], yc1 = ys[g + 8];
                 const uint32_t eo = sm + C::O_EPBUF + epar * (TU * EROW * 4);
@@ -796,8 +796,8 @@ __global__ void __launch_bounds__(NT, 1) wn_lat_kernel(const WnParams p, const u
                     if (lane == 0) {
                         int fbk = y;
                         if (b < B) {
-                            p.yOut[(size_t)b * p.N + t] = y;
-                            if (p.forced) fbk = p.forced[(size_t)b * p.N + t];
+                            p.yOut[(size_t)b * p.N + (t - p.origin)] = y;
+                            if (p.forced) fbk = p.forced[(size_t)b * p.N + (t - p.origin)];
                         } else fbk = 128;
                         ys[TU + 2 * w + r] = ys[2 * w + r];
                         ys[2 * w + r] = fbk;
@@ -1153,8 +1153,8 @@ __global__ void __launch_bounds__(NTC, 1) wn_lat2_kernel(const WnParams p, const
             for (int i = 0; i < C::NSK; i++) sk[i][0] = sk[i][1] = sk[i][2] = sk[i][3] = 0.f;
             uint32_t pc = 0, hcnt = 0;
             for (int t = t_begin; t < t_end; t++) {
-                const float sel0 = (2 * w + 0 + tile * TU) < B ? p.sel[(size_t)t * B + tile * TU + 2 * w] : 0.5f;
-                const float sel1 = (2 * w + 1 + tile * TU) < B ? p.sel[(size_t)t * B + tile * TU + 2 * w + 1] : 0.5f;
+                const float sel0 = (2 * w + 0 + tile * TU) < B ? p.sel[(size_t)(t - p.origin) * B +tile * TU + 2 * w] : 0.5f;
+                const float sel1 = (2 * w + 1 + tile * TU) < B ? p.sel[(size_t)(t - p.origin) * B +tile * TU + 2 * w + 1] : 0.5f;
                 for (int l = 0; l < L; l++, pc++, hcnt++) {
                     const uint32_t hb = sm + M::T_HBUF + (hcnt & 1) * 2048;
                     mbar_wait_a(s_hfull + 8 * (hcnt & 1), (hcnt >> 1) & 1);
@@ -1308,8 +1308,8 @@ __global__ void __launch_bounds__(NTC, 1) wn_lat2_kernel(const WnParams p, const
                         if (lane == 0) {
                             int fbk = y;
                             if (b < B) {
-                                p.yOut[(size_t)b * p.N + t] = y;
-                                if (p.forced) fbk = p.forced[(size_t)b * p.N + t];
+                                p.yOut[(size_t)b * p.N + (t - p.origin)] = y;
+                                if (p.forced) fbk = p.forced[(size_t)b * p.N + (t - p.origin)];
                             } else fbk = 128;
                             const int yold = ys[2 * w + r];
                             ys[TU + 2 * w + r] = yold;
@@ -1362,7 +1362,7 @@ __global__ void __launch_bounds__(NTC, 1) wn_lat2_kernel(const WnParams p, const
             // NPS = 8 slots: a slot is staged again five steps after its use, and the weight ring (4 pieces) keeps the warps within four.
             StepIt itp{t_begin, 0, t_begin % slots};
             uint32_t pcnt = 0;
-            const unsigned char* cptr = static_cast<const unsigned char*>(p.Lh) + (size_t)tile * 4096 + (size_t)(w * 32 + lane) * 16 + (size_t)t_begin * L * cstride;
+            const unsigned char* cptr = static_cast<const unsigned char*>(p.Lh) + (size_t)tile * 4096 + (size_t)(w * 32 + lane) * 16 + (size_t)(t_begin - p.origin) * L * cstride;
             auto stage = [&]() {
                 const uint32_t slot = pcnt & (M::NPS - 1);
                 if (itp.t < t_end) cp_async16(s_cond + slot * 4096, cptr);

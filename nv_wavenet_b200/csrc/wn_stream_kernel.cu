@@ -294,7 +294,7 @@ __global__ void __launch_bounds__(Shape<R, S>::NT + (RING ? 32 : 0), 1) wn_strea
     };
     auto lh_at = [&](int t, int l, int idx) -> const TD* {
         const int b = idx / (2 * R), row = idx % (2 * R);
-        return Lh + (((size_t)t * L + l) * B + (b0 + b)) * (2 * R) + row;
+        return Lh + (((size_t)(t - p.origin) * L + l) * B + (b0 + b)) * (2 * R) + row;
     };
 
     // prefetch registers for (t = init, l = 0)
@@ -535,7 +535,7 @@ __global__ void __launch_bounds__(Shape<R, S>::NT + (RING ? 32 : 0), 1) wn_strea
             }
             SYNC();
             if (tid < BT) {
-                const float sel = p.sel[(size_t)t * B + b0 + tid];
+                const float sel = p.sel[(size_t)(t - p.origin) * B +b0 + tid];
                 const float* pr = ex + tid * A;
                 float cs = 0.f;
                 int y = -1;
@@ -544,8 +544,8 @@ __global__ void __launch_bounds__(Shape<R, S>::NT + (RING ? 32 : 0), 1) wn_strea
                     if (sel < cs) { y = a; break; }
                 }
                 if (y < 0) y = A - 1;       // the reference asserts here (reference.cpp:119)
-                p.yOut[(size_t)(b0 + tid) * p.N + t] = y;
-                const int fb = p.forced ? p.forced[(size_t)(b0 + tid) * p.N + t] : y;
+                p.yOut[(size_t)(b0 + tid) * p.N + (t - p.origin)] = y;
+                const int fb = p.forced ? p.forced[(size_t)(b0 + tid) * p.N + (t - p.origin)] : y;
                 ysm[tid * 2] = ysm[tid * 2 + 1];
                 ysm[tid * 2 + 1] = fb;
             }
@@ -572,7 +572,7 @@ __global__ void __launch_bounds__(Shape<R, S>::NT + (RING ? 32 : 0), 1) wn_strea
                     if (lane >= o) inc += v;
                 }
                 const float total = __shfl_sync(0xffffffffu, inc, 31);
-                const float target = p.sel[(size_t)t * B + b0 + warp] * total;
+                const float target = p.sel[(size_t)(t - p.origin) * B +b0 + warp] * total;
                 const unsigned hit = __ballot_sync(0xffffffffu, target < inc);
                 int y = A - 1;
                 if (hit) {
@@ -592,8 +592,8 @@ __global__ void __launch_bounds__(Shape<R, S>::NT + (RING ? 32 : 0), 1) wn_strea
                     for (int j = 0; j < per; j++) p.P[(size_t)(b0 + warp) * A + lane * per + j] = e[j] * inv;
                 }
                 if (lane == 0) {
-                    p.yOut[(size_t)(b0 + warp) * p.N + t] = y;
-                    const int fb = p.forced ? p.forced[(size_t)(b0 + warp) * p.N + t] : y;
+                    p.yOut[(size_t)(b0 + warp) * p.N + (t - p.origin)] = y;
+                    const int fb = p.forced ? p.forced[(size_t)(b0 + warp) * p.N + (t - p.origin)] : y;
                     ysm[warp * 2] = ysm[warp * 2 + 1];
                     ysm[warp * 2 + 1] = fb;
                 }

@@ -298,7 +298,7 @@ __global__ void __launch_bounds__(NT, 1) wn_tc_kernel(const WnParams p, const un
     const size_t c_bpad = cond_bpad(B, TU);
     const unsigned char* gcond = static_cast<const unsigned char*>(p.Lh);
     auto cond_ptr = [&](int t, int l, int half) -> const unsigned char* {
-        return gcond + (((size_t)t * L + l) * c_bpad + (size_t)tile * TU) * 256 + (size_t)half * c_bytes;
+        return gcond + (((size_t)(t - p.origin) * L + l) * c_bpad + (size_t)tile * TU) * 256 + (size_t)half * c_bytes;
     };
 
     // debug timeline: role r (0 epilogue thread 0, 1 MMA issuer, 2 producer) appends (tag << 48 | clock) words
@@ -341,9 +341,10 @@ __global__ void __launch_bounds__(NT, 1) wn_tc_kernel(const WnParams p, const un
                 if (elect_one()) {
                     mbar_arrive_expect_tx(&cond_full[cbuf], 2 * c_bytes);
                     tma_load_1d(t_cond + (size_t)cbuf * CB, cond_ptr(t, l, 0), 2 * c_bytes, &cond_full[cbuf]);   // both halves are contiguous
-                    // pull the tiles a few layers ahead from HBM into L2
-                    int tl = t * L + l + 4;
-                    if (tl < t_end * L) tma_prefetch_l2(cond_ptr(tl / L, tl % L, 0), 2 * c_bytes);
+                    // pull the tiles a few layers ahead from HBM into L2 (sample and layer kept apart: t * L overflows an int
+                    // at sample indices a windowed engine reaches)
+                    const int ta = t + (l + 4) / L, la = (l + 4) % L;
+                    if (ta < t_end) tma_prefetch_l2(cond_ptr(ta, la, 0), 2 * c_bytes);
                 }
                 __syncwarp();
                 g_cond++;
@@ -861,7 +862,7 @@ __global__ void __launch_bounds__(NT, 1) wn_tc_kernel(const WnParams p, const un
         for (int t = t_begin; t < t_end; t++) {
             const bool dump = p.dump && (t == t_end - 1);
             tr_on = (t == tr_t);
-            const float sel = valid ? __ldg(p.sel + (size_t)t * B + b) : 0.5f;
+            const float sel = valid ? __ldg(p.sel + (size_t)(t - p.origin) * B + b) : 0.5f;
             if (!FUSED) prestore(0);                                    // D1[0] <- Lh[t][0] + Bh (Dza of the previous sample is consumed)
             // ---------------- embedding: x0 = tanh(embPrev[yPrev] + embCur[yCur])   (reference.cpp:42-57)
             if (wv) {
@@ -1176,7 +1177,7 @@ __global__ void __launch_bounds__(NT, 1) wn_tc_kernel(const WnParams p, const un
                         if (!found && target < run) { yy = c0 + 2 * j + 1; found = true; }
                     }
                     s_y[u] = yy;
-                    if (valid) p.yOut[(size_t)b * p.N + t] = yy;
+                    if (valid) p.yOut[(size_t)b * p.N + (t - p.origin)] = yy;
                 }
                 if (dump && valid) {
                     const float inv = fme / total;
@@ -1190,7 +1191,7 @@ __global__ void __launch_bounds__(NT, 1) wn_tc_kernel(const WnParams p, const un
             epi_bar();
             if (wv) y = s_y[u];
             if (valid) {
-                const int fb = p.forced ? p.forced[(size_t)b * p.N + t] : y;
+                const int fb = p.forced ? p.forced[(size_t)b * p.N + (t - p.origin)] : y;
                 yp = yc;
                 yc = fb;
             }

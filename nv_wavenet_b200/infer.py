@@ -44,16 +44,23 @@ def _stream(stream):
 
 class NVWavenetInfer:
     """nvWavenetInfer(numLayers, maxDilation, batchSize, numSamples, impl=0, tanhEmbed=True)
-    with the template parameters (precision, R, S, A) as keyword arguments."""
+    with the template parameters (precision, R, S, A) as keyword arguments.
+
+    `window=W` with `num_samples=None` creates a windowed engine (nvwn_create_windowed): its stores hold W samples, sample t in
+    slot t % W, so it generates utterances of any length in fixed device memory.  Sample ranges are absolute; see
+    include/nvwn_b200.h for what a windowed engine accepts."""
 
     def __init__(self, num_layers, max_dilation, batch_size, num_samples, impl=AUTO, tanh_embed=True,
-                 *, R=64, S=128, A=256, dtype=FP32):
+                 *, R=64, S=128, A=256, dtype=FP32, window=None):
         self._l = _lib.lib()
-        self.L, self.max_dilation, self.B, self.N = num_layers, max_dilation, batch_size, num_samples
+        if (num_samples is None) == (window is None):
+            raise ValueError("give num_samples (a full engine) or window (a windowed engine), not both")
+        self.L, self.max_dilation, self.B, self.N, self.W = num_layers, max_dilation, batch_size, num_samples, window
         self.R, self.S, self.A, self.dtype = R, S, A, dtype
         h = C.c_void_p()
-        check(self._l.nvwn_create(C.byref(h), dtype, R, S, A, num_layers, max_dilation, batch_size, num_samples,
-                                  impl, int(bool(tanh_embed))), "nvwn_create")
+        create = self._l.nvwn_create if window is None else self._l.nvwn_create_windowed
+        check(create(C.byref(h), dtype, R, S, A, num_layers, max_dilation, batch_size, num_samples if window is None else window,
+                     impl, int(bool(tanh_embed))), "nvwn_create" if window is None else "nvwn_create_windowed")
         self._h = h
         self._samples_per_chunk = 0
 
@@ -97,6 +104,17 @@ class NVWavenetInfer:
     def set_selectors_random(self, seed, stream=None):
         """Selectors drawn on the device: counter-based (Philox-4x32-10, key = seed), see include/nvwn_b200.h."""
         check(self._l.nvwn_set_selectors_random(self._h, C.c_ulonglong(int(seed) & (2 ** 64 - 1)), _stream(stream)), "setSelectorsRandom")
+
+    def set_selectors_range(self, selectors, first_sample, num_samples, stream=None):
+        """Selectors of samples [first_sample, first_sample + num_samples) only: float32 [num_samples][B], host or device."""
+        s, k = _ptr(selectors, np.float32)
+        check(self._l.nvwn_set_selectors_range(self._h, s, first_sample, num_samples, _stream(stream)), "setSelectorsRange")
+        return k
+
+    def set_selectors_random_range(self, seed, first_sample, num_samples, stream=None):
+        """The values set_selectors_random(seed) gives samples [first_sample, first_sample + num_samples), drawn for those only."""
+        check(self._l.nvwn_set_selectors_random_range(self._h, C.c_ulonglong(int(seed) & (2 ** 64 - 1)), first_sample, num_samples,
+                                                      _stream(stream)), "setSelectorsRandomRange")
 
     def set_conditioning(self, Lh, first_sample, num_samples, stream=None):
         a, k = _ptr(Lh, np.float32)
@@ -168,8 +186,12 @@ class NVWavenetInfer:
         mu-law decode (utils.mu_law_decode_numpy, mu_quantization = A) of yOut[:, offset:offset+size], as float32
         in [-1, 1] or, with int16=True, as `(MAX_WAV_VALUE * audio).astype('int16')`.  `out`: numpy array or torch
         tensor [B][size] of the matching dtype (a CUDA tensor is filled asynchronously on `stream`); allocated
-        (numpy) if None.  saturate=False keeps the reference's cast of the top code (+1.0 -> -32768)."""
-        size = self.N - offset if size is None else size
+        (numpy) if None.  saturate=False keeps the reference's cast of the top code (+1.0 -> -32768).  On a windowed engine
+        `offset` is an absolute sample index and `size` must be given."""
+        if size is None:
+            if self.W is not None:
+                raise ValueError("get_audio on a windowed engine needs `size`")
+            size = self.N - offset
         if out is None:
             out = np.empty((self.B, size), np.int16 if int16 else np.float32)
         if isinstance(out, np.ndarray):

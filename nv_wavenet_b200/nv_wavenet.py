@@ -10,6 +10,9 @@ frees it again on EVERY call) the object keeps a persistent engine per (batch, s
 infer() only sets the inputs.  Selectors: `seed=None` draws them like the reference (libc rand(), replayable with srand());
 an integer seed draws them on the device (counter-based Philox, include/nvwn_b200.h).
 
+`generate()` streams audio of any length from mel frames: a windowed engine (fixed device memory whatever the length), the
+conditioning produced on the device one chunk ahead on a side stream, and the mu-law decode on the device.
+
 Constructor arguments, accepted shapes, the appended unused residual layer and the memory layouts handed to the
 kernel are those of pytorch/nv_wavenet.py:55-196; the code is organised around one table of expected shapes.
 """
@@ -94,17 +97,17 @@ class NVWaveNet:
             self.layers.append((column_major(w[:, :, 0]), column_major(w[:, :, 1]), dilate_biases[l],
                                 column_major(res_weights[l]), res_biases[l], column_major(skip_weights[l]), skip_biases[l]))
         self.num_layers = n
-        self._engines = {}                               # (batch, samples, fp16) -> persistent NVWavenetInfer
+        self._engines = {}                               # (batch, samples, fp16, window) -> persistent NVWavenetInfer
         self.engines_created = 0
 
-    def _engine(self, batch_size, sample_count, fp16):
-        """The persistent engine for this problem size (created and loaded on first use)."""
+    def _engine(self, batch_size, sample_count, fp16, window=None):
+        """The persistent engine for this problem size (created and loaded on first use); a windowed one if `window` is given."""
         from .infer import NVWavenetInfer
-        key = (batch_size, sample_count, bool(fp16))
+        key = (batch_size, sample_count, bool(fp16), window)
         eng = self._engines.get(key)
         if eng is None:
             eng = NVWavenetInfer(self.num_layers, self.max_dilation, batch_size, sample_count, 0, bool(self.use_embed_tanh),
-                                 R=self.R, S=self.S, A=self.A, dtype=_lib.FP16 if fp16 else _lib.FP32)
+                                 R=self.R, S=self.S, A=self.A, dtype=_lib.FP16 if fp16 else _lib.FP32, window=window)
             f32 = lambda t: t.float().contiguous()
             eng.set_embeddings(f32(self.embedding_prev), f32(self.embedding_curr))
             for l, layer in enumerate(self.layers):
@@ -136,3 +139,50 @@ class NVWaveNet:
         eng.run(sample_count, batch_size, samples, dump_activations=False)
         torch.cuda.synchronize()
         return samples
+
+    def generate(self, features, upsample_weight, upsample_bias, cond_weight, cond_bias, stride, chunk=8000, seed=0, fp16=False):
+        """Streams the audio of mel frames `features` [B][C][T] chunk by chunk: yields (first_sample, audio) with `audio` an int16
+        CUDA tensor [B][n] (the reference's post-processing, saturate off), ordered on the current stream.
+
+        The upsampling and cond layers are those of set_conditioning_from_features (upsample_weight [C][C][window], cond_weight
+        [L*2R][C]).  One persistent windowed engine per (batch, chunk, precision) with a window of two chunks holds the utterance,
+        so device memory does not grow with T.  Chunk k+1's conditioning is produced on a side stream while chunk k generates;
+        it overwrites the slots of chunk k-1 only after that chunk's audio is decoded.  Selectors are the counter-based ones of
+        `seed`, so the audio equals infer(cond_input, seed=seed) on the same conditioning."""
+        B = features.size(0)
+        eng = self._engine(B, None, fp16, window=2 * chunk)
+        total = eng.cond_producer_load(features, upsample_weight, upsample_bias, cond_weight, cond_bias, stride)
+        eng.reset_history()
+        main, side = torch.cuda.current_stream(), torch.cuda.Stream()
+        starts = list(range(0, total, chunk))
+        produced, decoded = [], []
+
+        def produce(k):
+            s0 = starts[k]
+            if k == 0:
+                side.wait_stream(main)                                  # any earlier use of the engine on this stream
+            if k >= 2:
+                side.wait_event(decoded[k - 2])                         # chunk k takes the slots of chunk k - 2
+            eng.cond_producer_run(s0, min(chunk, total - s0), stream=side)
+            ev = torch.cuda.Event()
+            ev.record(side)
+            produced.append(ev)
+
+        produce(0)
+        for k, s0 in enumerate(starts):
+            n = min(chunk, total - s0)
+            if k + 1 < len(starts):
+                produce(k + 1)
+            eng.set_selectors_random_range(seed, s0, n, stream=main)
+            main.wait_event(produced[k])
+            eng._samples_per_chunk = n
+            try:
+                eng.run_partial(s0, total, B, None, 1, False, main)
+            finally:
+                eng._samples_per_chunk = 0
+            audio = torch.empty((B, n), dtype=torch.int16, device="cuda")
+            eng.get_audio(s0, n, int16=True, out=audio, stream=main)
+            ev = torch.cuda.Event()
+            ev.record(main)
+            decoded.append(ev)
+            yield s0, audio
